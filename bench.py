@@ -25,6 +25,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 S, C, V, N_HYP = 64, 32, 16, 8
@@ -363,9 +364,10 @@ def run_ours(args):
     ops.KernelTrace.reset(enabled=False)
     e0 = torch.cuda.Event(enable_timing=True); e1 = torch.cuda.Event(enable_timing=True)
     e0.record()
-    est.estimate(z_obj, target_dev, camera=hyp_full.to(dev))
+    timed_best = est.estimate(z_obj, target_dev, camera=hyp_full.to(dev))
     e1.record()
     barrier()
+    outputs = timed_outputs(timed_best, getattr(est, '_refiner', None)) if args.dump_outputs else None
     ms_total = max_over_ranks(e0.elapsed_time(e1))
     launches = ops.KernelTrace.launches
     ms_per_step = ms_total / args.steps
@@ -442,6 +444,10 @@ def run_ours(args):
         dist.destroy_process_group()
     if rank != 0:
         return
+    if outputs is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in outputs.items():
+            np.save(os.path.join(args.dump_outputs, f'{name}.npy'), a)
 
     # ---------------- roofline of the dominant kernel + per-kernel table ----------------
     peaks = measured_peaks()
@@ -519,6 +525,18 @@ def run_ours(args):
                       "views_per_gpu": (V + world - 1) // world, "fuser": "gru",
                       "note": "LatentFusionModel.build_latent_object, views sharded over the ranks (dist.py), max over ranks"}}
     print(json.dumps(line), flush=True)
+
+
+def timed_outputs(best, refiner):
+    """Host float32 copies of what the timed estimate() call computed: the ranked cameras it returns and, from its
+    last iteration, every hypothesis' rank loss, loss terms and updated camera parameters (this rank's hypotheses).
+    Every reduction on this path adds in a fixed order, so runs with the same arguments write the same bits."""
+    out = {'best_translation': best.translation, 'best_log_quaternion': best.log_quaternion}
+    if refiner is not None:
+        last = (int(refiner.slot) - 1) % refiner.chunk  # the slot advances after every replayed iteration
+        out.update(last_rank_loss=refiner.h_rank[last], last_loss_terms=refiner.h_terms[last],
+                   hyp_log_quaternion=refiner.lq, hyp_translation=refiner.tr, hyp_viewport=refiner.vp)
+    return {k: v.detach().float().cpu().numpy() for k, v in out.items()}
 
 
 def train_block(args, dev, rank, world, barrier, max_over_ranks, B=8, vin=16, vout=8):
@@ -620,7 +638,6 @@ def search_block(args, dev, rank, world, barrier, max_over_ranks, S4=128, C4=16,
     est.num_iters = 1                         # (the elite schedule keeps the config's 30-generation horizon)
     group = dist.group.WORLD if world > 1 else None
     torch.manual_seed(5)                      # every rank draws the same population
-    import numpy as np
     np.random.seed(5)
     est.estimate(z_obj, target, group=group)                      # warm-up generation
     est.num_iters = gens
@@ -710,7 +727,15 @@ def main():
     ap.add_argument('--no-strong', action='store_true', help='skip the configs[2] strong-scaling extra')
     ap.add_argument('--no-train', action='store_true', help='skip the configs[3] training-iteration extra')
     ap.add_argument('--no-search', action='store_true', help='skip the configs[4] coarse-search extra')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write what the timed path computed in its last step as DIR/<name>.npy (float32; with --gpus '
+                         '> 1, rank 0\'s hypotheses and the merged ranking); the inputs are seeded, so runs with the same '
+                         'arguments can be compared output for output')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'ours':
+        ap.error('--dump-outputs applies to --impl ours')
     args.warmup = max(args.warmup, 0)
     if args.hypotheses != N_HYP:
         globals()['N_HYP'] = args.hypotheses

@@ -252,31 +252,34 @@ int lf_refine_record(const float* terms /*[n][k]*/, int n, int k, const float* w
  *      :555-558 denormalize_depth; pose/estimation.py:70-118 default_pose_loss; pose/utils.py:81-117) ----
  * depth_logits, mask_logits [N][P][P] (the two heads of the Photographer); viewport [N][4] (x0,y0,x1,y1);
  * tz [N] camera translation z; target_depth / target_mask [height][width] (one target observation).
- * terms [N][4] = ov_depth, depth, iou, mask.  sums [N][8] is scratch carried from fwd to bwd. */
+ * terms [N][4] = ov_depth, depth, iou, mask.  sums [N][8] is scratch carried from fwd to bwd.  workspace is device
+ * scratch of lf_pose_loss_fwd_ws / lf_pose_loss_bwd_ws bytes: every reduction adds per-block or per-pixel partials in
+ * a fixed order (no atomics), so the same inputs give the same bits on every run. */
 typedef struct {
     int n, p;              /* hypotheses, crop side */
     int width, height;     /* full frame */
     float z_span, eps;     /* Camera.z_span; denormalize_depth eps (0.01) */
     /* layout of the logit maps and of tz, in floats; 0 = dense ([N][P][P] maps, tz[N]).  The decoder's fused heads write
      * channels-last logits [N][P][P][H]: depth_logits = base, mask_logits = base + 1, pix_stride = H, hyp_stride = P*P*H;
-     * tz = translation + 2 with tz_stride = 3.  The gradients use the layout of their inputs; with a non-dense layout
-     * lf_pose_loss_bwd does not zero-fill them (grad_depth_logits / grad_mask_logits when pix/hyp strides are given,
-     * grad_tz when tz_stride > 1): the caller passes zero-filled tensors. */
+     * tz = translation + 2 with tz_stride = 3.  The gradients use the layout of their inputs; lf_pose_loss_bwd writes
+     * every element of the two logit maps, of grad_viewport and the N entries of grad_tz, and nothing in between. */
     int pix_stride, hyp_stride, tz_stride;
 } lf_loss_desc;
 int lf_pose_loss_fwd(const lf_loss_desc* desc, const float* depth_logits, const float* mask_logits,
                      const float* viewport, const float* tz, const float* target_depth, const float* target_mask,
-                     float* sums, float* terms, void* stream);
+                     float* sums, float* terms, void* workspace, void* stream);
+int64_t lf_pose_loss_fwd_ws(const lf_loss_desc* desc);   /* bytes of workspace for lf_pose_loss_fwd / _search_fwd */
+int64_t lf_pose_loss_bwd_ws(const lf_loss_desc* desc);   /* bytes of workspace for lf_pose_loss_bwd */
 /* forward-only variant for the coarse search (CrossEntropyPoseEstimator: estimation.py:187-197 multiplies the crop's
  * metric depth by the crop's sigmoid(mask) before the loss pastes it into the frame); same outputs as lf_pose_loss_fwd */
 int lf_pose_loss_search_fwd(const lf_loss_desc* desc, const float* depth_logits, const float* mask_logits,
                             const float* viewport, const float* tz, const float* target_depth,
-                            const float* target_mask, float* sums, float* terms, void* stream);
+                            const float* target_mask, float* sums, float* terms, void* workspace, void* stream);
 int lf_pose_loss_bwd(const lf_loss_desc* desc, const float* depth_logits, const float* mask_logits,
                      const float* viewport, const float* tz, const float* target_depth, const float* target_mask,
                      const float* sums, const float* grad_terms /* [N][4] */,
                      float* grad_depth_logits, float* grad_mask_logits, float* grad_viewport /* [N][4] */,
-                     float* grad_tz /* [N] */, void* stream);
+                     float* grad_tz /* [N] */, void* workspace, void* stream);
 
 /* ---- wide 3x3x3 layers: weights streamed through shared memory (csrc/conv3d_ws.cu) ----
  * The same reference op as lf_conv3d_dz for the released network widths (tools/train/train.sh:37-46: 64/128/256-channel

@@ -99,9 +99,11 @@ _SIGNATURES = {
     'lf_adam_step': (c_int, [c_f32p] * 4 + [c_int, c_int, c_f32p, c_f32p, c_float, c_float, c_float, c_vp]),
     'lf_refine_record': (c_int, [c_f32p, c_int, c_int] + [c_f32p] * 11 + [c_vp, c_int, c_f32p, c_vp]),
     'lf_plateau_step': (c_int, [c_f32p] * 4 + [c_int, c_float, c_float, c_float, c_vp]),
-    'lf_pose_loss_fwd': (c_int, [ctypes.POINTER(LossDesc)] + [c_f32p] * 8 + [c_vp]),
-    'lf_pose_loss_search_fwd': (c_int, [ctypes.POINTER(LossDesc)] + [c_f32p] * 8 + [c_vp]),
-    'lf_pose_loss_bwd': (c_int, [ctypes.POINTER(LossDesc)] + [c_f32p] * 12 + [c_vp]),
+    'lf_pose_loss_fwd': (c_int, [ctypes.POINTER(LossDesc)] + [c_f32p] * 8 + [c_vp, c_vp]),
+    'lf_pose_loss_search_fwd': (c_int, [ctypes.POINTER(LossDesc)] + [c_f32p] * 8 + [c_vp, c_vp]),
+    'lf_pose_loss_bwd': (c_int, [ctypes.POINTER(LossDesc)] + [c_f32p] * 12 + [c_vp, c_vp]),
+    'lf_pose_loss_fwd_ws': (c_i64, [ctypes.POINTER(LossDesc)]),
+    'lf_pose_loss_bwd_ws': (c_i64, [ctypes.POINTER(LossDesc)]),
     'lf_conv_bwd_data_epi_supported': (c_int, [ctypes.POINTER(ConvDesc)]),
     'lf_conv_bwd_data_epi': (c_int, [ctypes.POINTER(ConvDesc), c_f32p, c_f32p, c_f32p, c_f32p, c_int, ctypes.c_float, c_int, c_f32p, c_vp]),
     'lf_heads_fwd': (c_int, [c_f32p, c_f32p, c_f32p, c_f32p, c_i64, c_int, c_int, ctypes.c_float, c_vp]),

@@ -7,7 +7,7 @@ namespace lf {
 // ---------------------------------------------------------------------------------------------
 // Interpolate (modules/__init__.py:18-33 -> F.interpolate(scale_factor, mode, align_corners=False)).
 //   nearest: src = floor(dst / scale)         linear: src = (dst + .5)/scale - .5, clamped at 0
-// Each output (or, in backward, each gradient) element is a tensor-product of <= 2 taps per axis.
+// Each output element is a tensor-product of <= 2 taps per axis; the backward gathers through the same taps.
 // ---------------------------------------------------------------------------------------------
 struct Tap { int i0, i1; float w0, w1; };
 
@@ -36,10 +36,9 @@ struct InterpGeom {
     int mode;
 };
 
-template <bool BWD, int VEC>
-__global__ void interp_kernel(const InterpGeom g, const float* __restrict__ src, float* __restrict__ dst) {
-    // forward: src = x, dst = y (gather).  backward: src = gy, dst = gx (scatter with reductions; gx zeroed).
-    // VEC = 4 when C % 4 == 0: one thread moves 4 channels with 128-bit loads/stores/reductions.
+template <int VEC>
+__global__ void interp_kernel(const InterpGeom g, const float* __restrict__ x, float* __restrict__ y) {
+    // VEC = 4 when C % 4 == 0: one thread moves 4 channels with 128-bit loads/stores.
     const int cv = g.c / VEC;
     const int64_t total = (int64_t)g.n * g.od * g.oh * g.ow * cv;
     for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < total; e += (int64_t)gridDim.x * blockDim.x) {
@@ -53,13 +52,9 @@ __global__ void interp_kernel(const InterpGeom g, const float* __restrict__ src,
         const Tap ty = axis_tap(oy, g.h, g.mode, g.fh);
         const Tap tx = axis_tap(ox, g.w, g.mode, g.fw);
         const int64_t base = (int64_t)n * g.d;
-        float acc[VEC], gv[VEC];
+        float acc[VEC];
 #pragma unroll
-        for (int j = 0; j < VEC; ++j) { acc[j] = 0.f; gv[j] = 0.f; }
-        if (BWD) {
-            if (VEC == 4) { const float4 t = ldg4(src + e * 4); gv[0] = t.x; gv[1] = t.y; gv[2] = t.z; gv[3] = t.w; }
-            else gv[0] = src[e];
-        }
+        for (int j = 0; j < VEC; ++j) acc[j] = 0.f;
 #pragma unroll
         for (int a = 0; a < 2; ++a) {
             const float wz = a ? tz.w1 : tz.w0; const int iz = a ? tz.i1 : tz.i0;
@@ -74,23 +69,71 @@ __global__ void interp_kernel(const InterpGeom g, const float* __restrict__ src,
                     if (wx == 0.f) continue;
                     const float wgt = wz * wy * wx;
                     const int64_t idx = (((base + iz) * g.h + iy) * g.w + ix) * g.c + c;
-                    if (BWD) {
-                        if (VEC == 4) atomicAdd(reinterpret_cast<float4*>(dst + idx),
-                                                make_float4(gv[0] * wgt, gv[1] * wgt, gv[2] * wgt, gv[3] * wgt));
-                        else atomicAdd(dst + idx, gv[0] * wgt);
-                    } else if (VEC == 4) {
-                        const float4 t = ldg4(src + idx);
+                    if (VEC == 4) {
+                        const float4 t = ldg4(x + idx);
                         acc[0] += wgt * t.x; acc[1] += wgt * t.y; acc[2] += wgt * t.z; acc[3] += wgt * t.w;
                     } else {
-                        acc[0] += wgt * src[idx];
+                        acc[0] += wgt * x[idx];
                     }
                 }
             }
         }
-        if (!BWD) {
-            if (VEC == 4) *reinterpret_cast<float4*>(dst + e * 4) = make_float4(acc[0], acc[1], acc[2], acc[3]);
-            else dst[e] = acc[0];
+        if (VEC == 4) *reinterpret_cast<float4*>(y + e * 4) = make_float4(acc[0], acc[1], acc[2], acc[3]);
+        else y[e] = acc[0];
+    }
+}
+
+// The weight output o gives input index i along one axis through its forward taps (both taps count when a border
+// clamp makes them coincide).  Only outputs in gather_lo(i) .. gather_hi(i) can reach i: 2i-1 .. 2i+2 when upsampling
+// (the linear stencil; nearest uses 2i, 2i+1), i/2 when downsampling (taps 2o, 2o+1 linear, 2o nearest).
+__device__ __forceinline__ float tap_weight(int o, int i, int in_size, int mode, int factor) {
+    const Tap t = axis_tap(o, in_size, mode, factor);
+    return (t.i0 == i ? t.w0 : 0.f) + (t.i1 == i ? t.w1 : 0.f);
+}
+__device__ __forceinline__ int gather_lo(int i, int factor) { return max(factor == 1 ? i : (factor > 0 ? 2 * i - 1 : i / 2), 0); }
+__device__ __forceinline__ int gather_hi(int i, int out_size, int factor) {
+    return min(factor == 1 ? i : (factor > 0 ? 2 * i + 2 : i / 2), out_size - 1);
+}
+
+// Backward as a gather: each element of gx sums its gradient contributions in a fixed order, so the result does not
+// depend on scheduling (a scatter with float atomics would add them in a different order on every run).
+template <int VEC>
+__global__ void interp_bwd_kernel(const InterpGeom g, const float* __restrict__ gy, float* __restrict__ gx) {
+    const int cv = g.c / VEC;
+    const int64_t total = (int64_t)g.n * g.d * g.h * g.w * cv;
+    for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < total; e += (int64_t)gridDim.x * blockDim.x) {
+        int64_t r = e;
+        const int c = (int)(r % cv) * VEC; r /= cv;
+        const int ix = (int)(r % g.w); r /= g.w;
+        const int iy = (int)(r % g.h); r /= g.h;
+        const int iz = (int)(r % g.d); r /= g.d;
+        const int n = (int)r;
+        const int64_t base = (int64_t)n * g.od;
+        float acc[VEC];
+#pragma unroll
+        for (int j = 0; j < VEC; ++j) acc[j] = 0.f;
+        for (int oz = gather_lo(iz, g.fd); oz <= gather_hi(iz, g.od, g.fd); ++oz) {
+            const float wz = tap_weight(oz, iz, g.d, g.mode, g.fd);
+            if (wz == 0.f) continue;
+            for (int oy = gather_lo(iy, g.fh); oy <= gather_hi(iy, g.oh, g.fh); ++oy) {
+                const float wy = tap_weight(oy, iy, g.h, g.mode, g.fh);
+                if (wy == 0.f) continue;
+                for (int ox = gather_lo(ix, g.fw); ox <= gather_hi(ix, g.ow, g.fw); ++ox) {
+                    const float wx = tap_weight(ox, ix, g.w, g.mode, g.fw);
+                    if (wx == 0.f) continue;
+                    const float wgt = wz * wy * wx;
+                    const int64_t idx = (((base + oz) * g.oh + oy) * g.ow + ox) * g.c + c;
+                    if (VEC == 4) {
+                        const float4 t = ldg4(gy + idx);
+                        acc[0] += wgt * t.x; acc[1] += wgt * t.y; acc[2] += wgt * t.z; acc[3] += wgt * t.w;
+                    } else {
+                        acc[0] += wgt * gy[idx];
+                    }
+                }
+            }
         }
+        if (VEC == 4) *reinterpret_cast<float4*>(gx + e * 4) = make_float4(acc[0], acc[1], acc[2], acc[3]);
+        else gx[e] = acc[0];
     }
 }
 
@@ -326,8 +369,8 @@ extern "C" int lf_interp_fwd(const float* x, float* y, int ndim, int n, int d, i
     if (int e = interp_geom(g, ndim, n, d, h, w, c, mode, factor)) return e;
     LF_CHECK_ARG(x && y, "interp: null pointer");
     const int64_t total = (int64_t)g.n * g.od * g.oh * g.ow * g.c;
-    if ((g.c & 3) == 0) interp_kernel<false, 4><<<ew_grid(total / 4), 256, 0, (cudaStream_t)stream>>>(g, x, y);
-    else interp_kernel<false, 1><<<ew_grid(total), 256, 0, (cudaStream_t)stream>>>(g, x, y);
+    if ((g.c & 3) == 0) interp_kernel<4><<<ew_grid(total / 4), 256, 0, (cudaStream_t)stream>>>(g, x, y);
+    else interp_kernel<1><<<ew_grid(total), 256, 0, (cudaStream_t)stream>>>(g, x, y);
     LF_RETURN_LAUNCH();
 }
 
@@ -336,10 +379,9 @@ extern "C" int lf_interp_bwd(const float* gy, float* gx, int ndim, int n, int d,
     InterpGeom g;
     if (int e = interp_geom(g, ndim, n, d, h, w, c, mode, factor)) return e;
     LF_CHECK_ARG(gy && gx, "interp: null pointer");
-    const int64_t total = (int64_t)g.n * g.od * g.oh * g.ow * g.c;
-    cudaMemsetAsync(gx, 0, sizeof(float) * (size_t)g.n * g.d * g.h * g.w * g.c, (cudaStream_t)stream);
-    if ((g.c & 3) == 0) interp_kernel<true, 4><<<ew_grid(total / 4), 256, 0, (cudaStream_t)stream>>>(g, gy, gx);
-    else interp_kernel<true, 1><<<ew_grid(total), 256, 0, (cudaStream_t)stream>>>(g, gy, gx);
+    const int64_t total = (int64_t)g.n * g.d * g.h * g.w * g.c;
+    if ((g.c & 3) == 0) interp_bwd_kernel<4><<<ew_grid(total / 4), 256, 0, (cudaStream_t)stream>>>(g, gy, gx);
+    else interp_bwd_kernel<1><<<ew_grid(total), 256, 0, (cudaStream_t)stream>>>(g, gy, gx);
     LF_RETURN_LAUNCH();
 }
 

@@ -8,9 +8,11 @@
 //   default_pose_loss (pose/estimation.py:70-118) + pose/utils.py:81-117 reductions
 // i.e. ~100 elementwise/reduction launches over [N,1,480,640] intermediates plus two
 // grid_sampler_2d_backward launches that serialise on border-pixel atomics (1.5 ms each on B200),
-// by two passes over the full frame that never materialise a full-frame tensor:
+// by two passes over the full frame:
 //   pass 1: per-hypothesis partial sums  ->  the four loss terms
-//   pass 2: d(terms)/d(depth logits, mask logits, viewport, translation_z)
+//   pass 2: d(terms)/d(depth logits, mask logits, viewport, translation_z): per-pixel gradients, gathered into the
+//           crop maps by a row and a column pass (the taps are separable), every sum in a fixed order
+
 #include "common.cuh"
 
 namespace lf {
@@ -45,26 +47,43 @@ __device__ __forceinline__ float clip_coord(float g, int P, float& mult) {
     return ix;
 }
 
+// one axis of a full-frame pixel's sample in the crop: gx = (X - v0)/(v1 - v0)*2 - 1 (geometry.py:281-282)
+struct AxisSample {
+    int i0, i1, near;         // bilinear taps (i1 == i0 at the far border) and the nearest tap
+    int in;                   // whether the +1 tap is in range
+    float f, w0, w1;          // fraction, tap weights (w1 = 0 at the far border)
+    float m;                  // d(ix)/d(unclipped ix): 1 inside, 0 where border-clamped
+    float ix;                 // the sample coordinate in [0, P-1]
+};
+
+__device__ __forceinline__ AxisSample axis_sample(float X, float v0, float v1, int P) {
+    AxisSample a;
+    const float gx = (X - v0) / (v1 - v0) * 2.f - 1.f;
+    float ix = clip_coord(gx, P, a.m);
+    // degenerate optimised viewport (zero width / NaN): the reference only propagates NaNs; keep the indices in range
+    if (!isfinite(ix)) { ix = 0.f; a.m = 0.f; }
+    a.ix = ix;
+    a.near = (int)nearbyintf(ix);
+    const float f0 = floorf(ix);
+    a.i0 = (int)f0;
+    a.f = ix - f0;
+    a.in = (a.i0 + 1 < P);
+    a.i1 = a.in ? a.i0 + 1 : a.i0;
+    a.w0 = 1.f - a.f;
+    a.w1 = a.in ? a.f : 0.f;
+    return a;
+}
+
 __device__ __forceinline__ PixelSample make_sample(float X, float Y, const float* vp, int P, int ps) {
     PixelSample s;
-    const float vw = vp[2] - vp[0], vh = vp[3] - vp[1];
-    const float gx = (X - vp[0]) / vw * 2.f - 1.f;       // geometry.py:281-282
-    const float gy = (Y - vp[1]) / vh * 2.f - 1.f;
-    float ix = clip_coord(gx, P, s.mx), iy = clip_coord(gy, P, s.my);
-    // degenerate optimised viewport (zero width / NaN): the reference only propagates NaNs; keep the indices in range
-    if (!isfinite(ix)) { ix = 0.f; s.mx = 0.f; }
-    if (!isfinite(iy)) { iy = 0.f; s.my = 0.f; }
-    const int xn = (int)nearbyintf(ix), yn = (int)nearbyintf(iy);
-    s.near_idx = (yn * P + xn) * ps;
-    const float fx0 = floorf(ix), fy0 = floorf(iy);
-    const int x0 = (int)fx0, y0 = (int)fy0;
-    s.fx = ix - fx0; s.fy = iy - fy0;
-    s.x0in = (x0 + 1 < P); s.y0in = (y0 + 1 < P);
-    const int x1 = s.x0in ? x0 + 1 : x0, y1 = s.y0in ? y0 + 1 : y0;
-    s.i00 = (y0 * P + x0) * ps; s.i01 = (y0 * P + x1) * ps; s.i10 = (y1 * P + x0) * ps; s.i11 = (y1 * P + x1) * ps;
-    const float wx1 = s.x0in ? s.fx : 0.f, wy1 = s.y0in ? s.fy : 0.f;
-    const float wx0 = 1.f - s.fx, wy0 = 1.f - s.fy;
-    s.w00 = wx0 * wy0; s.w01 = wx1 * wy0; s.w10 = wx0 * wy1; s.w11 = wx1 * wy1;
+    const AxisSample ax = axis_sample(X, vp[0], vp[2], P), ay = axis_sample(Y, vp[1], vp[3], P);
+    s.mx = ax.m; s.my = ay.m;
+    s.near_idx = (ay.near * P + ax.near) * ps;
+    s.fx = ax.f; s.fy = ay.f;
+    s.x0in = ax.in; s.y0in = ay.in;
+    s.i00 = (ay.i0 * P + ax.i0) * ps; s.i01 = (ay.i0 * P + ax.i1) * ps;
+    s.i10 = (ay.i1 * P + ax.i0) * ps; s.i11 = (ay.i1 * P + ax.i1) * ps;
+    s.w00 = ax.w0 * ay.w0; s.w01 = ax.w1 * ay.w0; s.w10 = ax.w0 * ay.w1; s.w11 = ax.w1 * ay.w1;
     return s;
 }
 
@@ -93,7 +112,7 @@ __device__ __forceinline__ PixelTerms eval_pixel(const PixelSample& s, const flo
 __global__ void __launch_bounds__(256)
 pose_loss_sums_kernel(const LossGeom g, const float* __restrict__ dlog, const float* __restrict__ mlog,
                       const float* __restrict__ vp, const float* __restrict__ tz,
-                      const float* __restrict__ tdepth, const float* __restrict__ tmask, float* __restrict__ sums) {
+                      const float* __restrict__ tdepth, const float* __restrict__ tmask, float* __restrict__ part) {
     const int n = blockIdx.y;
     const int HW = g.width * g.height;
     const float* dl = dlog + (size_t)n * g.hs;
@@ -122,17 +141,28 @@ pose_loss_sums_kernel(const LossGeom g, const float* __restrict__ dlog, const fl
     if (threadIdx.x < kSums) {
         float r = 0.f;
         for (int w = 0; w < 8; ++w) r += red[w][threadIdx.x];
-        atomicAdd(sums + n * 8 + threadIdx.x, r);
+        part[((size_t)n * gridDim.x + blockIdx.x) * kSums + threadIdx.x] = r;
     }
 }
 
-// terms[n] = (ov_depth, depth, iou, mask); sums[n][6] = sum target_mask*valid (set by the first kernel below)
-__global__ void pose_loss_terms_kernel(const LossGeom g, const float* __restrict__ sums, float* __restrict__ terms) {
+// Adds the per-block partials of the two kernels around it in block order (no atomics: the same inputs give the same
+// bits on every run) into sums[n][0..6], sums[n][6] = sum target_mask*valid, then
+// terms[n] = (ov_depth, depth, iou, mask).
+__global__ void pose_loss_terms_kernel(const LossGeom g, const float* __restrict__ part, int bx,
+                                       const float* __restrict__ tpart, int tb, float* __restrict__ sums,
+                                       float* __restrict__ terms) {
     const int n = blockIdx.x * blockDim.x + threadIdx.x;
     if (n >= g.n) return;
-    const float* s = sums + n * 8;
+    float* s = sums + n * 8;
+    for (int k = 0; k < kSums; ++k) {
+        float r = 0.f;
+        for (int b = 0; b < bx; ++b) r += part[((size_t)n * bx + b) * kSums + k];
+        s[k] = r;
+    }
+    float G = 0.f;
+    for (int b = 0; b < tb; ++b) G += tpart[b];
+    s[6] = G;
     const float HW = (float)(g.width * g.height);
-    const float G = s[6];
     const float U = s[3] + G - s[4];
     terms[n * 4 + 0] = fmaxf(s[1], 1e-5f) / fmaxf(s[2], 1e-4f);            // pose/utils.py:111-117
     terms[n * 4 + 1] = s[0] / HW;
@@ -141,7 +171,7 @@ __global__ void pose_loss_terms_kernel(const LossGeom g, const float* __restrict
 }
 
 __global__ void __launch_bounds__(256)
-target_sum_kernel(const LossGeom g, const float* __restrict__ tdepth, const float* __restrict__ tmask, float* __restrict__ sums) {
+target_sum_kernel(const LossGeom g, const float* __restrict__ tdepth, const float* __restrict__ tmask, float* __restrict__ tpart) {
     const int HW = g.width * g.height;
     float a = 0.f;
     for (int px = blockIdx.x * blockDim.x + threadIdx.x; px < HW; px += gridDim.x * blockDim.x) {
@@ -155,18 +185,7 @@ target_sum_kernel(const LossGeom g, const float* __restrict__ tdepth, const floa
     if (threadIdx.x == 0) {
         float r = 0.f;
         for (int w = 0; w < 8; ++w) r += red[w];
-        for (int n = 0; n < g.n; ++n) atomicAdd(sums + n * 8 + 6, r);
-    }
-}
-
-// one atomic per warp when every lane hits the same address (pixels clamped to the crop border), else per lane
-__device__ __forceinline__ void warp_atomic_add(float* base, int idx, float v) {
-    const int idx0 = __shfl_sync(0xffffffffu, idx, 0);
-    if (__all_sync(0xffffffffu, idx == idx0)) {
-        v = warp_sum(v);
-        if ((threadIdx.x & 31) == 0 && v != 0.f) atomicAdd(base + idx0, v);
-    } else if (v != 0.f) {
-        atomicAdd(base + idx, v);
+        tpart[blockIdx.x] = r;
     }
 }
 
@@ -175,13 +194,13 @@ pose_loss_bwd_kernel(const LossGeom g, const float* __restrict__ dlog, const flo
                      const float* __restrict__ vp, const float* __restrict__ tz,
                      const float* __restrict__ tdepth, const float* __restrict__ tmask,
                      const float* __restrict__ sums, const float* __restrict__ gterms,
-                     float* __restrict__ g_dl, float* __restrict__ g_ml, float* __restrict__ g_vp, float* __restrict__ g_tz) {
+                     float2* __restrict__ g_pix, float* __restrict__ vpart) {
+    // pass 1 of the backward: every full-frame pixel's d(total)/d(sampled mask logit, depth logit) -> g_pix[n][px], and
+    // this block's share of d/d(viewport, tz) -> vpart; pose_loss_rows/cols_kernel gather g_pix into the crop maps
     const int n = blockIdx.y;
     const int HW = g.width * g.height;
     const float* dl = dlog + (size_t)n * g.hs;
     const float* ml = mlog + (size_t)n * g.hs;
-    float* gdl = g_dl + (size_t)n * g.hs;
-    float* gml = g_ml + (size_t)n * g.hs;
     const float base = tz[n * g.tzs] + g.base_off;
     const float* s = sums + n * 8;
     const float fHW = (float)HW;
@@ -201,14 +220,10 @@ pose_loss_bwd_kernel(const LossGeom g, const float* __restrict__ dlog, const flo
     const float half_p = (float)g.p * 0.5f;            // d ix / d gx
 
     float a_tz = 0.f, a_vp[4] = {0.f, 0.f, 0.f, 0.f};
-    // full warps only: the aggregation helper uses warp-wide votes
-    const int HW_pad = (HW + 31) & ~31;
-    for (int px = blockIdx.x * blockDim.x + threadIdx.x; px < HW_pad; px += gridDim.x * blockDim.x) {
-        const bool live = px < HW;
-        const int pc = live ? px : HW - 1;
-        const int Y = pc / g.width, X = pc - Y * g.width;
+    for (int px = blockIdx.x * blockDim.x + threadIdx.x; px < HW; px += gridDim.x * blockDim.x) {
+        const int Y = px / g.width, X = px - Y * g.width;
         const PixelSample smp = make_sample((float)X, (float)Y, vp + 4 * n, g.p, g.ps);
-        const PixelTerms t = eval_pixel(smp, dl, ml, tdepth[pc], tmask[pc], g.range, base);
+        const PixelTerms t = eval_pixel(smp, dl, ml, tdepth[px], tmask[px], g.range, base);
         float d_dl1 = dA + dB * t.pm * t.tm;
         float d_pm = dB * t.dl1 * t.tm + dC * t.tm + dD + dE * t.tm * t.valid;
         const float diff = t.pd - t.td;
@@ -216,16 +231,10 @@ pose_loss_bwd_kernel(const LossGeom g, const float* __restrict__ dlog, const flo
         const float d_pd = d_dl1 * t.valid * sgn;
         const float d_z = d_pd * t.pm;
         d_pm += d_pd * t.z;
-        float d_ml = d_pm * t.pm * (1.f - t.pm) + dF * (t.pm - t.tm);
-        float d_dlog = d_z * (1.f - t.th * t.th) * 0.5f * t.gate * g.range;
-        if (!live) { d_ml = 0.f; d_dlog = 0.f; }
-        a_tz += live ? d_z : 0.f;
-        // bilinear taps of the mask logits
-        warp_atomic_add(gml, smp.i00, d_ml * smp.w00);
-        warp_atomic_add(gml, smp.i01, d_ml * smp.w01);
-        warp_atomic_add(gml, smp.i10, d_ml * smp.w10);
-        warp_atomic_add(gml, smp.i11, d_ml * smp.w11);
-        warp_atomic_add(gdl, smp.near_idx, d_dlog);
+        const float d_ml = d_pm * t.pm * (1.f - t.pm) + dF * (t.pm - t.tm);
+        const float d_dlog = d_z * (1.f - t.th * t.th) * 0.5f * t.gate * g.range;
+        a_tz += d_z;
+        g_pix[(size_t)n * HW + px] = make_float2(d_ml, d_dlog);
         // d(ml_full)/d(ix, iy) -> viewport (ATen grid_sampler_2d_backward: gix uses the in-range taps only)
         const float m00 = ml[smp.i00], m01 = smp.x0in ? ml[smp.i01] : 0.f;
         const float m10 = smp.y0in ? ml[smp.i10] : 0.f, m11 = (smp.x0in && smp.y0in) ? ml[smp.i11] : 0.f;
@@ -255,8 +264,116 @@ pose_loss_bwd_kernel(const LossGeom g, const float* __restrict__ dlog, const flo
     if (threadIdx.x < 5) {
         float r = 0.f;
         for (int w = 0; w < 8; ++w) r += red[w][threadIdx.x];
-        if (threadIdx.x < 4) atomicAdd(g_vp + 4 * n + threadIdx.x, r);
-        else atomicAdd(g_tz + n * g.tzs, r);
+        vpart[((size_t)n * gridDim.x + blockIdx.x) * 5 + threadIdx.x] = r;
+    }
+}
+
+// The pixels whose sample along one axis has its first bilinear tap in [t0, t1]: a contiguous range [lo, hi), as the
+// tap is non-decreasing in the pixel coordinate for a viewport of positive extent (clamping and float rounding are
+// monotone).  Any other viewport (flipped, empty, NaN) scans the whole axis.
+__device__ __forceinline__ void tap_range(int t0, int t1, float v0, float v1, int P, int len, int& lo, int& hi) {
+    if (!((v1 - v0) > 0.f)) { lo = 0; hi = len; return; }
+    auto first = [&](int t) {               // first pixel whose tap is >= t
+        int a = 0, b = len;
+        while (a < b) {
+            const int mid = (a + b) >> 1;
+            if (axis_sample((float)mid, v0, v1, P).i0 >= t) b = mid; else a = mid + 1;
+        }
+        return a;
+    };
+    lo = first(t0);
+    hi = first(t1 + 1);
+}
+
+// The pixels at the two ends of an axis whose sample is clamped to the crop border (coordinate 0, resp. P-1) give their
+// whole value to the border texel, for the bilinear and the nearest tap alike.  A warp adds them up cooperatively
+// (lane-strided partials, then a fixed shuffle tree), and the per-texel loops cover only the pixels in between:
+// [lo_in, hi_in).  A viewport of non-positive extent keeps the full per-texel scans.
+struct BorderSums { int lo_in, hi_in; float2 left, right; };
+
+__device__ __forceinline__ BorderSums border_sums(const float2* src, int64_t stride, int len, float v0, float v1, int P) {
+    BorderSums b;
+    b.lo_in = 0; b.hi_in = len;
+    b.left = b.right = make_float2(0.f, 0.f);
+    if (!((v1 - v0) > 0.f)) return b;
+    auto first = [&](float t, bool strict) {        // first pixel whose coordinate is > t (strict) or >= t
+        int a = 0, e = len;
+        while (a < e) {
+            const int mid = (a + e) >> 1;
+            const float ix = axis_sample((float)mid, v0, v1, P).ix;
+            if (strict ? ix > t : ix >= t) e = mid; else a = mid + 1;
+        }
+        return a;
+    };
+    b.lo_in = first(0.f, true);
+    b.hi_in = first((float)(P - 1), false);
+    const int lane = threadIdx.x & 31;
+    float lx = 0.f, ly = 0.f, rx = 0.f, ry = 0.f;
+    for (int i = lane; i < b.lo_in; i += 32) { const float2 v = src[i * stride]; lx += v.x; ly += v.y; }
+    for (int i = b.hi_in + lane; i < len; i += 32) { const float2 v = src[i * stride]; rx += v.x; ry += v.y; }
+    b.left = make_float2(warp_sum(lx), warp_sum(ly));
+    b.right = make_float2(warp_sum(rx), warp_sum(ry));
+    return b;
+}
+
+// Sum over the in-between pixels of one texel: mask-logit values weighted by the texel's bilinear tap weight, and the
+// depth-logit values of the pixels whose nearest tap is the texel, in increasing pixel order.
+__device__ __forceinline__ float2 texel_sum(const float2* src, int64_t stride, int len, float v0, float v1, int P, int t,
+                                            const BorderSums& b) {
+    int lo, hi;
+    tap_range(t - 1, t, v0, v1, P, len, lo, hi);
+    lo = max(lo, b.lo_in);
+    hi = min(hi, b.hi_in);
+    float sml = 0.f, sdl = 0.f;
+    for (int i = lo; i < hi; ++i) {
+        const AxisSample a = axis_sample((float)i, v0, v1, P);
+        const float w = (a.i0 == t ? a.w0 : 0.f) + (a.i1 == t ? a.w1 : 0.f);
+        const float2 v = src[i * stride];
+        sml += v.x * w;
+        if (a.near == t) sdl += v.y;
+    }
+    if (t == 0) { sml += b.left.x; sdl += b.left.y; }
+    if (t == P - 1) { sml += b.right.x; sdl += b.right.y; }
+    return make_float2(sml, sdl);
+}
+
+// pass 2, one warp per (n, Y): rows[n][Y][tx] = x-gather of row Y of the per-pixel gradients into the crop columns.
+__global__ void __launch_bounds__(256)
+pose_loss_rows_kernel(const LossGeom g, const float* __restrict__ vp, const float2* __restrict__ g_pix,
+                      float2* __restrict__ rows) {
+    const int64_t row = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    if (row >= (int64_t)g.n * g.height) return;              // (whole warps)
+    const int n = (int)(row / g.height);
+    const float v0 = vp[4 * n], v1 = vp[4 * n + 2];
+    const float2* src = g_pix + row * g.width;
+    const BorderSums b = border_sums(src, 1, g.width, v0, v1, g.p);
+    for (int tx = threadIdx.x & 31; tx < g.p; tx += 32)
+        rows[row * g.p + tx] = texel_sum(src, 1, g.width, v0, v1, g.p, tx, b);
+}
+
+// pass 3, one warp per (n, tx): the y-gather of column tx of `rows` into the crop maps, written to every texel in the
+// inputs' layout; block 0 of each hypothesis adds the viewport / tz partials in block order.
+__global__ void __launch_bounds__(256)
+pose_loss_cols_kernel(const LossGeom g, const float* __restrict__ vp, const float2* __restrict__ rows,
+                      const float* __restrict__ vpart, int bx, float* __restrict__ g_dl, float* __restrict__ g_ml,
+                      float* __restrict__ g_vp, float* __restrict__ g_tz) {
+    const int n = blockIdx.y;
+    if (blockIdx.x == 0 && threadIdx.x < 5) {
+        float r = 0.f;
+        for (int b = 0; b < bx; ++b) r += vpart[((size_t)n * bx + b) * 5 + threadIdx.x];
+        if (threadIdx.x < 4) g_vp[4 * n + threadIdx.x] = r;
+        else g_tz[n * g.tzs] = r;
+    }
+    const int tx = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    if (tx >= g.p) return;                                    // (whole warps)
+    const float v0 = vp[4 * n + 1], v1 = vp[4 * n + 3];
+    const float2* src = rows + (size_t)n * g.height * g.p + tx;
+    const BorderSums b = border_sums(src, g.p, g.height, v0, v1, g.p);
+    for (int ty = threadIdx.x & 31; ty < g.p; ty += 32) {
+        const float2 v = texel_sum(src, g.p, g.height, v0, v1, g.p, ty, b);
+        const size_t e = (size_t)n * g.hs + (size_t)(ty * g.p + tx) * g.ps;
+        g_ml[e] = v.x;
+        g_dl[e] = v.y;
     }
 }
 
@@ -290,70 +407,97 @@ static int loss_geom(const lf_loss_desc* d, LossGeom& g) {
     return LF_OK;
 }
 
+// Workspaces (no atomics anywhere, so that the same inputs give the same bits on every run):
+//   forward : per-block partial sums of the loss kernel [n][bx][6] and of the target kernel [tb]
+//   backward: per-pixel gradients [n][H][W] float2, row sums [n][H][P] float2, per-block viewport/tz partials [n][bx][5]
+static int target_blocks(int HW) { return min(2 * sm_count(), (HW + 255) / 256); }
+
+static int64_t fwd_ws_floats(const LossGeom& g) {
+    const int HW = g.width * g.height;
+    return (int64_t)g.n * blocks_x(pose_loss_sums_kernel, g.n, HW) * kSums + target_blocks(HW);
+}
+
+static int64_t bwd_ws_floats(const LossGeom& g) {
+    const int HW = g.width * g.height;
+    return 2 * (int64_t)g.n * HW + 2 * (int64_t)g.n * g.height * g.p + (int64_t)g.n * blocks_x(pose_loss_bwd_kernel, g.n, HW) * 5;
+}
+
+static int loss_fwd(const LossGeom& g, const float* depth_logits, const float* mask_logits, const float* viewport,
+                    const float* tz, const float* target_depth, const float* target_mask, float* sums, float* terms,
+                    void* workspace, cudaStream_t st) {
+    const int HW = g.width * g.height;
+    const int bx = blocks_x(pose_loss_sums_kernel, g.n, HW), tb = target_blocks(HW);
+    float* part = (float*)workspace;
+    float* tpart = part + (size_t)g.n * bx * kSums;
+    target_sum_kernel<<<tb, 256, 0, st>>>(g, target_depth, target_mask, tpart);
+    pose_loss_sums_kernel<<<dim3(bx, g.n), 256, 0, st>>>(g, depth_logits, mask_logits, viewport, tz, target_depth, target_mask, part);
+    pose_loss_terms_kernel<<<(g.n + 63) / 64, 64, 0, st>>>(g, part, bx, tpart, tb, sums, terms);
+    LF_RETURN_LAUNCH();
+}
+
 }  // namespace lf
 
 using namespace lf;
 
-extern "C" int lf_pose_loss_fwd(const lf_loss_desc* desc, const float* depth_logits, const float* mask_logits,
-                                const float* viewport, const float* tz, const float* target_depth,
-                                const float* target_mask, float* sums, float* terms, void* stream) {
+extern "C" int64_t lf_pose_loss_fwd_ws(const lf_loss_desc* desc) {
     LossGeom g;
     if (int e = loss_geom(desc, g)) return e;
-    LF_CHECK_ARG(depth_logits && mask_logits && viewport && tz && target_depth && target_mask && sums && terms,
+    return 4 * fwd_ws_floats(g);
+}
+
+extern "C" int64_t lf_pose_loss_bwd_ws(const lf_loss_desc* desc) {
+    LossGeom g;
+    if (int e = loss_geom(desc, g)) return e;
+    return 4 * bwd_ws_floats(g);
+}
+
+extern "C" int lf_pose_loss_fwd(const lf_loss_desc* desc, const float* depth_logits, const float* mask_logits,
+                                const float* viewport, const float* tz, const float* target_depth,
+                                const float* target_mask, float* sums, float* terms, void* workspace, void* stream) {
+    LossGeom g;
+    if (int e = loss_geom(desc, g)) return e;
+    LF_CHECK_ARG(depth_logits && mask_logits && viewport && tz && target_depth && target_mask && sums && terms && workspace,
                  "pose_loss_fwd: null pointer");
-    cudaStream_t st = (cudaStream_t)stream;
-    cudaMemsetAsync(sums, 0, sizeof(float) * 8 * g.n, st);
-    const int HW = g.width * g.height;
-    const int bx = blocks_x(pose_loss_sums_kernel, g.n, HW);
-    target_sum_kernel<<<min(2 * sm_count(), (HW + 255) / 256), 256, 0, st>>>(g, target_depth, target_mask, sums);
-    pose_loss_sums_kernel<<<dim3(bx, g.n), 256, 0, st>>>(g, depth_logits, mask_logits, viewport, tz, target_depth, target_mask, sums);
-    pose_loss_terms_kernel<<<(g.n + 63) / 64, 64, 0, st>>>(g, sums, terms);
-    LF_RETURN_LAUNCH();
+    return loss_fwd(g, depth_logits, mask_logits, viewport, tz, target_depth, target_mask, sums, terms, workspace,
+                    (cudaStream_t)stream);
 }
 
 // Forward-only scoring for the coarse pose search (CrossEntropyPoseEstimator, reference estimation.py:187-197 +
 // :70-118): same four terms, with the search's extra crop-space mask factor on the rendered depth.
 extern "C" int lf_pose_loss_search_fwd(const lf_loss_desc* desc, const float* depth_logits, const float* mask_logits,
                                        const float* viewport, const float* tz, const float* target_depth,
-                                       const float* target_mask, float* sums, float* terms, void* stream) {
+                                       const float* target_mask, float* sums, float* terms, void* workspace,
+                                       void* stream) {
     LossGeom g;
     if (int e = loss_geom(desc, g)) return e;
     g.premask = 1;
-    LF_CHECK_ARG(depth_logits && mask_logits && viewport && tz && target_depth && target_mask && sums && terms,
+    LF_CHECK_ARG(depth_logits && mask_logits && viewport && tz && target_depth && target_mask && sums && terms && workspace,
                  "pose_loss_search_fwd: null pointer");
-    cudaStream_t st = (cudaStream_t)stream;
-    cudaMemsetAsync(sums, 0, sizeof(float) * 8 * g.n, st);
-    const int HW = g.width * g.height;
-    const int bx = blocks_x(pose_loss_sums_kernel, g.n, HW);
-    target_sum_kernel<<<min(2 * sm_count(), (HW + 255) / 256), 256, 0, st>>>(g, target_depth, target_mask, sums);
-    pose_loss_sums_kernel<<<dim3(bx, g.n), 256, 0, st>>>(g, depth_logits, mask_logits, viewport, tz, target_depth, target_mask, sums);
-    pose_loss_terms_kernel<<<(g.n + 63) / 64, 64, 0, st>>>(g, sums, terms);
-    LF_RETURN_LAUNCH();
+    return loss_fwd(g, depth_logits, mask_logits, viewport, tz, target_depth, target_mask, sums, terms, workspace,
+                    (cudaStream_t)stream);
 }
 
 extern "C" int lf_pose_loss_bwd(const lf_loss_desc* desc, const float* depth_logits, const float* mask_logits,
                                 const float* viewport, const float* tz, const float* target_depth,
                                 const float* target_mask, const float* sums, const float* grad_terms,
                                 float* grad_depth_logits, float* grad_mask_logits, float* grad_viewport,
-                                float* grad_tz, void* stream) {
+                                float* grad_tz, void* workspace, void* stream) {
     LossGeom g;
     if (int e = loss_geom(desc, g)) return e;
     LF_CHECK_ARG(depth_logits && mask_logits && viewport && tz && target_depth && target_mask && sums && grad_terms &&
-                 grad_depth_logits && grad_mask_logits && grad_viewport && grad_tz, "pose_loss_bwd: null pointer");
+                 grad_depth_logits && grad_mask_logits && grad_viewport && grad_tz && workspace,
+                 "pose_loss_bwd: null pointer");
     cudaStream_t st = (cudaStream_t)stream;
-    // dense layout: the gradients are zero-filled here; strided layout (maps interleaved in one tensor, tz a column of
-    // the translation): the caller passes zero-filled tensors of the inputs' layout
-    if (g.ps == 1 && g.hs == g.p * g.p) {
-        const size_t crop = sizeof(float) * (size_t)g.n * g.p * g.p;
-        cudaMemsetAsync(grad_depth_logits, 0, crop, st);
-        cudaMemsetAsync(grad_mask_logits, 0, crop, st);
-    }
-    cudaMemsetAsync(grad_viewport, 0, sizeof(float) * 4 * g.n, st);
-    if (g.tzs == 1) cudaMemsetAsync(grad_tz, 0, sizeof(float) * g.n, st);
     const int HW = g.width * g.height;
     const int bx = blocks_x(pose_loss_bwd_kernel, g.n, HW);
+    float2* g_pix = (float2*)workspace;
+    float2* rows = g_pix + (size_t)g.n * HW;
+    float* vpart = (float*)(rows + (size_t)g.n * g.height * g.p);
     pose_loss_bwd_kernel<<<dim3(bx, g.n), 256, 0, st>>>(g, depth_logits, mask_logits, viewport, tz, target_depth,
-                                                      target_mask, sums, grad_terms, grad_depth_logits,
-                                                      grad_mask_logits, grad_viewport, grad_tz);
+                                                      target_mask, sums, grad_terms, g_pix, vpart);
+    pose_loss_rows_kernel<<<(unsigned)(((int64_t)g.n * g.height * 32 + 255) / 256), 256, 0, st>>>(g, viewport, g_pix, rows);
+    pose_loss_cols_kernel<<<dim3((g.p * 32 + 255) / 256, g.n), 256, 0, st>>>(g, viewport, rows, vpart, bx,
+                                                                            grad_depth_logits, grad_mask_logits,
+                                                                            grad_viewport, grad_tz);
     LF_RETURN_LAUNCH();
 }

@@ -1109,6 +1109,14 @@ def depth_sum(x):
 # ------------------------------------------------------------------------------------------------
 # fused pose-loss head
 # ------------------------------------------------------------------------------------------------
+def _loss_ws(query, desc, device):
+    """device workspace of the pose-loss head (lf_pose_loss_fwd_ws / lf_pose_loss_bwd_ws bytes)"""
+    nbytes = query(ctypes.byref(desc))
+    if nbytes < 0:
+        L.check(int(nbytes), 'pose_loss workspace')
+    return torch.empty((nbytes + 3) // 4, device=device)
+
+
 class _PoseLoss(torch.autograd.Function):
     """interpret_logits + denormalize_depth + uncrop x2 + default_pose_loss terms in two full-frame passes.
     Returns terms [N,4] = (ov_depth, depth, iou, mask); differentiable w.r.t. the two logit maps, the
@@ -1127,8 +1135,9 @@ class _PoseLoss(torch.autograd.Function):
         desc = L.LossDesc(n, p, width, height, float(z_span), float(eps))
         sums = torch.empty(n, 8, device=dl.device)
         terms = torch.empty(n, 4, device=dl.device)
+        ws = _loss_ws(L.lib().lf_pose_loss_fwd_ws, desc, dl.device)
         _call('lf_pose_loss_fwd', L.lib().lf_pose_loss_fwd,
-              (ctypes.byref(desc), _p(dl), _p(ml), _p(vp), _p(tzc), _p(td), _p(tm), _p(sums), _p(terms), _stream()),
+              (ctypes.byref(desc), _p(dl), _p(ml), _p(vp), _p(tzc), _p(td), _p(tm), _p(sums), _p(terms), _p(ws), _stream()),
               kernels=3)
         ctx.save_for_backward(dl, ml, vp, tzc, td, tm, sums)
         ctx.cfg = (n, p, width, height, float(z_span), float(eps), tuple(depth_logits.shape), tuple(mask_logits.shape))
@@ -1143,9 +1152,10 @@ class _PoseLoss(torch.autograd.Function):
         g_dl, g_ml = torch.empty_like(dl), torch.empty_like(ml)
         g_vp, g_tz = torch.empty_like(vp), torch.empty_like(tzc)
         gt = gterms.float().contiguous()
+        ws = _loss_ws(L.lib().lf_pose_loss_bwd_ws, desc, dl.device)
         _call('lf_pose_loss_bwd', L.lib().lf_pose_loss_bwd,
               (ctypes.byref(desc), _p(dl), _p(ml), _p(vp), _p(tzc), _p(td), _p(tm), _p(sums), _p(gt),
-               _p(g_dl), _p(g_ml), _p(g_vp), _p(g_tz), _stream()))
+               _p(g_dl), _p(g_ml), _p(g_vp), _p(g_tz), _p(ws), _stream()), kernels=3)
         return g_dl.view(dshape), g_ml.view(mshape), g_vp, g_tz, None, None, None, None, None, None
 
 
@@ -1167,8 +1177,10 @@ class _PoseLossPacked(torch.autograd.Function):
         sums = torch.empty(n, 8, device=lg.device)
         terms = torch.empty(n, 4, device=lg.device)
         base = lg.data_ptr()
+        ws = _loss_ws(L.lib().lf_pose_loss_fwd_ws, desc, lg.device)
         _call('lf_pose_loss_fwd', L.lib().lf_pose_loss_fwd,
-              (ctypes.byref(desc), base, base + 4, _p(vp), tr.data_ptr() + 8, _p(td), _p(tm), _p(sums), _p(terms), _stream()),
+              (ctypes.byref(desc), base, base + 4, _p(vp), tr.data_ptr() + 8, _p(td), _p(tm), _p(sums), _p(terms), _p(ws),
+               _stream()),
               kernels=3)
         ctx.save_for_backward(lg, vp, tr, td, tm, sums)
         ctx.cfg = (n, hh, p, width, height, float(z_span), float(eps))
@@ -1181,13 +1193,14 @@ class _PoseLossPacked(torch.autograd.Function):
         n, hh, p, width, height, z_span, eps = ctx.cfg
         desc = L.LossDesc(n, p, width, height, z_span, eps, hh, p * p * hh, 3)
         g_lg = torch.zeros_like(lg)                       # (same channels-last strides)
-        g_tr = torch.zeros_like(tr)
+        g_tr = torch.zeros_like(tr)                       # (the kernel writes its z column only)
         g_vp = torch.empty_like(vp)
         gt = gterms.float().contiguous()
         base, gbase = lg.data_ptr(), g_lg.data_ptr()
+        ws = _loss_ws(L.lib().lf_pose_loss_bwd_ws, desc, lg.device)
         _call('lf_pose_loss_bwd', L.lib().lf_pose_loss_bwd,
               (ctypes.byref(desc), base, base + 4, _p(vp), tr.data_ptr() + 8, _p(td), _p(tm), _p(sums), _p(gt),
-               gbase, gbase + 4, _p(g_vp), g_tr.data_ptr() + 8, _stream()))
+               gbase, gbase + 4, _p(g_vp), g_tr.data_ptr() + 8, _p(ws), _stream()), kernels=3)
         return g_lg, g_vp, g_tr, None, None, None, None, None, None
 
 
@@ -1220,10 +1233,11 @@ def pose_search_terms(depth_logits, mask_logits, viewport, tz, target_depth, tar
     dl, ml = depth_logits.float().contiguous().view(n, p, p), mask_logits.float().contiguous().view(n, p, p)
     desc = L.LossDesc(n, p, width, height, float(z_span), float(eps))
     sums, terms = torch.empty(n, 8, device=dl.device), torch.empty(n, 4, device=dl.device)
+    ws = _loss_ws(L.lib().lf_pose_loss_fwd_ws, desc, dl.device)
     _call('lf_pose_loss_search_fwd', L.lib().lf_pose_loss_search_fwd,
           (ctypes.byref(desc), _p(dl), _p(ml), _p(viewport.float().contiguous()), _p(tz.float().contiguous()),
            _p(target_depth.float().contiguous().view(height, width)), _p(target_mask.float().contiguous().view(height, width)),
-           _p(sums), _p(terms), _stream()), kernels=3)
+           _p(sums), _p(terms), _p(ws), _stream()), kernels=3)
     return terms
 
 

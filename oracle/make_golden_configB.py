@@ -7,7 +7,8 @@ hypotheses are independent, so two pin the composition as well as eight).
     python oracle/make_golden_configB.py        # authoring container only (needs /root/reference)
 
 Writes tests/golden/configB_s64_c32.npz:
-  * the reference-format Photographer state_dict (random N(0,1) weights, seed 0; 278k floats),
+  * digests of the reference-format Photographer state_dict (random N(0,1) weights, seed 0; 278k floats), which
+    the tests draw again rather than read,
   * the hypothesis cameras, the target observation's generator parameters,
   * depth/mask logits, a strided sample of the projected latent, the four pose-loss terms,
   * camera gradients of (1.0*depth + 0.3*ov_depth) [configs/adam_quick.toml] in fp32 — the reference as shipped —
@@ -31,6 +32,7 @@ sys.path.insert(0, os.path.dirname(HERE))
 warnings.filterwarnings('ignore')
 
 from oracle import ref_import  # noqa: E402
+from tests import parity_helpers as ph  # noqa: E402
 
 ref_import.install()
 
@@ -130,8 +132,9 @@ def main():
     g['meta'] = np.array(json.dumps(dict(S=S, C=C, N=N, camera_dist=camera_dist, arch_photographer=arch_p,
                                          weights=WEIGHTS, z_obj='make_cube(smooth)', smooth=SMOOTH,
                                          target=dict(cy=251.5, cx=315.4, radius=45.0), torch=torch.__version__)))
-    for k, v in photographer.state_dict().items():
-        g[f'photographer/{k}'] = npy(v)
+    # the weights are drawn again by the tests (tests/parity_helpers.py, recipe 'configB'), checked against these digests
+    g['regenerated'] = np.array(json.dumps(dict(recipe='configB', digests={
+        f'photographer/{k}': ph.digest(npy(v)) for k, v in photographer.state_dict().items()})))
     for k in ('intrinsic', 'log_quaternion', 'translation', 'viewport'):
         g[f'hyp_cam.{k}'] = npy(getattr(hyp, k))
         g[f'gt_cam.{k}'] = npy(getattr(gt_full, k))

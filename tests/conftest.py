@@ -1,8 +1,6 @@
-import json
 import os
 import sys
 
-import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -14,31 +12,8 @@ def pytest_configure(config):
     config.addinivalue_line('markers', 'gpu: needs a CUDA device (run on the B200 box)')
 
 
-class Golden:
-    """Read-only view of tests/golden/lfsynth_s16_c8.npz (made by oracle/make_golden.py from the
-    unmodified reference)."""
-
-    def __init__(self, path):
-        self._z = np.load(path)
-        self.meta = json.loads(str(self._z['meta']))
-
-    def __getitem__(self, key):
-        import torch
-        return torch.from_numpy(np.array(self._z[key]))
-
-    def keys(self):
-        return self._z.files
-
-    def state_dict(self, prefix):
-        import torch
-        p = prefix + '/'
-        return {k[len(p):]: torch.from_numpy(np.array(self._z[k])) for k in self._z.files
-                if k.startswith(p)}
-
-    def cam(self, prefix):
-        return {k: self[f'{prefix}.{k}'] for k in ('intrinsic', 'log_quaternion', 'translation', 'viewport')}
-
-
 @pytest.fixture(scope='session')
 def golden():
-    return Golden(os.path.join(ROOT, 'tests', 'golden', 'lfsynth_s16_c8.npz'))
+    """tests/golden/lfsynth_s16_c8.npz (made by oracle/make_golden.py from the unmodified reference)."""
+    from tests import parity_helpers as ph
+    return ph.Golden(ph.GOLDEN)

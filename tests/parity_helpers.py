@@ -1,4 +1,5 @@
 """Shared helpers for the parity tests and ``__graft_entry__.smoke()`` (test infrastructure)."""
+import hashlib
 import json
 import os
 
@@ -12,13 +13,93 @@ GOLDEN = os.path.join(ROOT, 'tests', 'golden', 'lfsynth_s16_c8.npz')
 OUT_TOL = dict(atol=1e-4, rtol=1e-3)
 GRAD_TOL = dict(atol=2e-4, rtol=2e-3)
 
+# A golden output too large to store whole keeps every SAMPLE_STRIDE-th element of its flattened values.  The stride
+# is prime, so it is coprime with every extent and the sample covers all positions along each axis.
+SAMPLE_STRIDE = 7
+
+
+def sample(a):
+    """The stored sample of a large output (numpy array or tensor)."""
+    return a.reshape(-1)[::SAMPLE_STRIDE]
+
+
+def digest(a):
+    """Short SHA-256 of an array's dtype, shape and bytes: pins the arrays a golden file regenerates instead of
+    storing."""
+    a = np.ascontiguousarray(a)
+    h = hashlib.sha256(f'{a.dtype.str}{a.shape}'.encode())
+    h.update(a.tobytes())
+    return h.hexdigest()[:16]
+
+
+def reference_init(nets, seed):
+    """Draw the weights of product networks exactly as the reference's constructors draw the same architectures after
+    torch.manual_seed(seed), then the non-zero biases the golden scripts draw.  Each reference equalised convolution
+    wraps an nn.ConvNd, whose own init (kaiming_uniform_: one uniform draw per weight) is overwritten by N(0, 1); the
+    biases are then drawn N(0, 0.1), network by network."""
+    from latentfusion_b200.modules.equalized import Equalized
+    torch.manual_seed(seed)
+    with torch.no_grad():
+        for net in nets:
+            for m in net.modules():
+                if isinstance(m, Equalized):
+                    w = m.module.weight
+                    torch.empty_like(w).uniform_()
+                    w.normal_(0, 1)
+        for net in nets:
+            for k, p in net.named_parameters():
+                if k.endswith('bias'):
+                    p.normal_(0, 0.1)
+
+
+def _regenerate_lfsynth(meta):
+    """oracle/make_golden.py's networks (seed 0), reference views (seed 11) and resampler inputs (seed 13)."""
+    from latentfusion_b200.recon import fusion, models
+    S, C, V, N = meta['S'], meta['C'], meta['V'], meta['N']
+    nets = {'sculptor': models.Sculptor(**meta['arch_sculptor']),
+            'fuser': fusion.get_fuser('gru', in_channels=C, cube_size=1.0),
+            'photographer': models.Photographer(**meta['arch_photographer'])}
+    reference_init(nets.values(), seed=0)
+    out = {f'{name}/{k}': v.numpy() for name, net in nets.items() for k, v in net.state_dict().items()}
+    torch.manual_seed(11)
+    out['color'] = (torch.rand(1, V, 3, 2 * S, 2 * S) * 2 - 1).numpy()
+    torch.manual_seed(13)
+    for k, n in (('o2c.vol', 1), ('o2c.w', N), ('c2o.vol', V), ('c2o.w', V)):
+        out[k] = torch.randn(n, 5, 12, 12, 12).numpy()
+    return out
+
+
+def _regenerate_config_b(meta):
+    """oracle/make_golden_configB.py's Photographer (seed 0)."""
+    from latentfusion_b200.recon import models
+    photographer = models.Photographer(**meta['arch_photographer'])
+    reference_init([photographer], seed=0)
+    return {f'photographer/{k}': v.numpy() for k, v in photographer.state_dict().items()}
+
+
+_REGENERATE = {'lfsynth': _regenerate_lfsynth, 'configB': _regenerate_config_b}
+
 
 class Golden:
+    """Read-only view of a tests/golden/*.npz file.  Seeded inputs and weights that a file lists under `regenerated`
+    are drawn again here and must match the digests of what the reference was run with; outputs stored as a sample
+    are compared through `sampled`."""
+
     def __init__(self, path=GOLDEN):
         self._z = np.load(path)
         self.meta = json.loads(str(self._z['meta']))
+        self._regen = {}
+        if 'regenerated' in self._z.files:
+            spec = json.loads(str(self._z['regenerated']))
+            self._regen = _REGENERATE[spec['recipe']](self.meta)
+            assert set(self._regen) == set(spec['digests']), \
+                f'{path}: regenerated keys differ: {sorted(set(self._regen) ^ set(spec["digests"]))}'
+            bad = [k for k, d in spec['digests'].items() if digest(self._regen[k]) != d]
+            assert not bad, f'{path}: regenerated arrays differ from the ones the reference was run with: {bad}'
 
     def __getitem__(self, key):
+        if key in self._regen:
+            return torch.from_numpy(self._regen[key].copy())
         return torch.from_numpy(np.array(self._z[key]))
 
     def text(self, key):
@@ -26,7 +107,13 @@ class Golden:
 
     def state_dict(self, prefix):
         p = prefix + '/'
-        return {k[len(p):]: torch.from_numpy(np.array(self._z[k])) for k in self._z.files if k.startswith(p)}
+        return {k[len(p):]: self[k] for k in (*self._z.files, *self._regen) if k.startswith(p)}
+
+    def sampled(self, key, ours):
+        """(ours, golden) on the stored sample of output `key`, after checking that `ours` has the full shape."""
+        shape = tuple(int(n) for n in self._z[f'{key}.shape'])
+        assert tuple(ours.shape) == shape, f'{key}: shape {tuple(ours.shape)} != {shape}'
+        return sample(ours), self[f'{key}.sample']
 
     def cam(self, prefix):
         return {k: self[f'{prefix}.{k}'] for k in ('intrinsic', 'log_quaternion', 'translation', 'viewport')}

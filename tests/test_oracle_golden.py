@@ -70,11 +70,11 @@ def test_sculptor_and_fusers(golden):
     with torch.no_grad():
         x = torch.cat((color.flatten(0, 1), mask.flatten(0, 1) * 2 - 1), dim=1)
         z, z_cam_mid, _ = O.sculptor_forward(sd, arch, x, cam)
-        torch.testing.assert_close(z, golden['z_views'], **TOL)
-        torch.testing.assert_close(z_cam_mid[0], golden['z_cam_mid0'], **TOL)
+        torch.testing.assert_close(*golden.sampled('z_views', z), **TOL)
+        torch.testing.assert_close(*golden.sampled('z_cam_mid0', z_cam_mid[0]), **TOL)
         zv = z.view(1, -1, *z.shape[1:])
         for kind in ('max', 'mean', 'median', 'abs_max'):
-            torch.testing.assert_close(O.fuse(f'pool:{kind}', zv), golden[f'z_obj_pool_{kind}'], **TOL)
+            torch.testing.assert_close(*golden.sampled(f'z_obj_pool_{kind}', O.fuse(f'pool:{kind}', zv)), **TOL)
         zg = O.sculptor_encode(sd, arch, 'gru', golden.state_dict('fuser'), cam, color, mask)
         torch.testing.assert_close(zg, golden['z_obj_gru'], atol=1e-4, rtol=1e-3)
 

@@ -2,7 +2,7 @@
 """Per-kernel micro-benchmark at BASELINE config-2 extents (dev tool; numbers quoted in profiles/ come
 from bench.py's live trace, this is for iterating on one kernel and for ncu captures).
 
-  python tools/kbench.py [--only resample|conv|all] [--iters 20] [--precision 0|1|2]
+  python tools/kbench.py [--only resample|conv|ibr|loss|all] [--iters 20] [--precision 0|1|2]
 """
 import argparse
 import json
@@ -145,6 +145,38 @@ def main():
         for role, name in enumerate(('producer(plane)', 'mma(step)', 'epilogue(step)')):
             rows = [(i, int(buf[role, i, 0] - t0), int(buf[role, i, 1] - t0)) for i in range(40) if buf[role, i, 0] > 0]
             print(name, ' '.join(f'{i}:[{a},{b}]' for i, a, b in rows[:20]))
+    if a.only in ('all', 'loss'):
+        # the fused pose-loss head at the refine shapes (N hypotheses, 2S x 2S crop, 640 x 480 frame), and the 2-D resize
+        # backward at the decoder's / encoder's shapes for N refine views and for the training step's 64 / 128 views
+        import ctypes
+        from latentfusion_b200 import _lib as L
+        P = 2 * S
+        torch.manual_seed(1)
+        base = torch.randn(N, P, P, 2, device=dev)              # the fused heads' channels-last logits [N,2,P,P]
+        vp0, tr0 = cam.viewport.detach().clone(), cam.translation.detach().clone()
+        yy, xx = torch.meshgrid(torch.arange(480.0, device=dev), torch.arange(640.0, device=dev), indexing='ij')
+        tm = (((yy - 251.5) ** 2 + (xx - 315.4) ** 2) <= 45.0 ** 2).float().view(1, 1, 480, 640)
+        td = tm * float(tr0[0, 2])
+        med, best = timeit(lambda: ops.pose_loss_terms_packed(base.permute(0, 3, 1, 2), vp0, tr0, td, tm, cam.z_span),
+                           a.iters, flush)
+        out['pose_loss_fwd'] = dict(ms=med, best_ms=best)
+        lg, vp, tr = base.clone().requires_grad_(True), vp0.clone().requires_grad_(True), tr0.clone().requires_grad_(True)
+        gt = torch.ones(N, 4, device=dev)
+
+        def loss_fwd_bwd():
+            ops.pose_loss_terms_packed(lg.permute(0, 3, 1, 2), vp, tr, td, tm, cam.z_span).backward(gt)
+        med2, best2 = timeit(loss_fwd_bwd, a.iters, flush)
+        out['pose_loss_fwd+bwd'] = dict(ms=med2, best_ms=best2, bwd_only_ms=med2 - med)
+        st = ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)
+        for name, n, hw, c, factor in (('up_32to64', N, 32, 64, 2), ('up_64to128', N, 64, 64, 2), ('down_128to64', N, 128, 32, -2),
+                                       ('train_up_32to64', 64, 32, 64, 2), ('train_up_64to128', 64, 64, 64, 2),
+                                       ('train_down_128to64', 128, 128, 32, -2)):
+            ohw = hw * 2 if factor > 0 else hw // 2
+            gy = torch.randn(n, ohw, ohw, c, device=dev)
+            gx = torch.empty(n, hw, hw, c, device=dev)
+            med, best = timeit(lambda: L.check(L.lib().lf_interp_bwd(ops._p(gy), ops._p(gx), 2, n, 1, hw, hw, c, 1, factor, st),
+                                               'interp_bwd'), a.iters, flush)
+            out[f'interp_bwd_bilinear[{name}]'] = dict(ms=med, best_ms=best, GBs=4 * (gy.numel() + gx.numel()) / med / 1e6)
     print(json.dumps(out, indent=1))
 
 
